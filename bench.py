@@ -2,7 +2,7 @@
 """bench.py -- V-cycles/s of the B200 AMG solve-phase engine on BASELINE.json's configurations.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg3|cfg2|cfg4|cfg5]
-                    [--grid G] [--configs cfg2,cfg5,cfg4]
+                    [--grid G] [--configs cfg2,cfg5,cfg4] [--dump-outputs DIR]
 
 Headline workload (config.workload): BASELINE.json configs[2] -- gallery.poisson((256,256,256)) 7-pt fp64,
 ruge_stuben_solver hierarchy (classical strength 0.25, RS splitting, classical interpolation), multi-colour
@@ -482,6 +482,22 @@ def ncu_traffic(kernel_key):
         return None
 
 
+DUMP_MAX_ENTRIES = 1 << 22       # 32 MB of float64: what --dump-outputs writes stays under 64 MB
+
+
+def dump_outputs(out_dir, x, norms2):
+    """--dump-outputs: what the timed amgb_solve_device call hands its caller, so that two builds run with the same
+    arguments (hence the same inputs) can be compared output for output.  x.npy is the iterate after the last timed
+    cycle (float64; above DUMP_MAX_ENTRIES entries a fixed sample at seeded positions, in index order) and
+    residual_norms_sq.npy the call's steps + 1 squared residual norms."""
+    os.makedirs(out_dir, exist_ok=True)
+    x = x.cpu().numpy()
+    if x.size > DUMP_MAX_ENTRIES:
+        x = x[np.sort(np.random.default_rng(SEED).choice(x.size, DUMP_MAX_ENTRIES, replace=False))]
+    np.save(os.path.join(out_dir, "x.npy"), x)
+    np.save(os.path.join(out_dir, "residual_norms_sq.npy"), norms2.cpu().numpy())
+
+
 def measure_config(name, grid, args, local, tstream, steps, warmup, cpu_sample, headline):
     """Everything bench.py reports for ONE workload on one GPU: device-resident V-cycles/s, e2e through the C ABI
     with host buffers, per-kernel roofline table, the reference's CPU path beside it and full-size parity."""
@@ -523,6 +539,8 @@ def measure_config(name, grid, args, local, tstream, steps, warmup, cpu_sample, 
     ms = e0.elapsed_time(e1)
     launches = ml.last_launches()
     res = np.sqrt(norms[:steps + 1].cpu().numpy())
+    if headline and args.dump_outputs:
+        dump_outputs(args.dump_outputs, x, norms[:steps + 1])
 
     # ---- end to end through the C ABI with host buffers (one cycle per call) ---------------
     nres, info = ctypes.c_int32(0), ctypes.c_int32(0)
@@ -672,7 +690,12 @@ def main():
                          "under 'configs' (value, e2e, roofline, cpu_baseline, parity_full_size each); '' = none")
     ap.add_argument("--configs-budget-s", type=float, default=480.0,
                     help="a configuration of --configs is skipped once this much wall time has been spent on them")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the headline workload's timed solve returned as "
+                         "DIR/<name>.npy (single GPU, --impl ours)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs is implemented for --impl ours on one GPU")
     WORKLOAD["name"] = args.workload
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     g = args.grid if args.grid is not None else DEFAULT_GRID[args.workload]

@@ -12,6 +12,9 @@ Run in the build container only (the GPU box has no /root/reference):
     printf 'Metadata-Version: 2.1\nName: pyamg\nVersion: 0.0.0+oracle\n' > $D/pyamg-0.0.0.dist-info/METADATA
     # 2. generate
     cd /root/repo && PYTHONPATH=/tmp/pyamg_ref python tests/golden/make_golden.py
+    # 3. the goldens of the tests that compare with the reference directly (tests/golden/reference/; they also
+    #    need oracle/_ref/libamg_ref.so, which build() compiles where the reference sources are present)
+    PYTHONPATH=<the reference build of step 1> python tests/golden/make_golden.py --reference-checks
 
 Every fixture is one .npz written by pyamg_b200.hierarchy_io.save_hierarchy: the hierarchy the
 reference built (operators, smoother closures' parameters, cached coarse pinv) plus, as extra
@@ -291,7 +294,136 @@ def main_widening():
     emit("cfg10_sa_bgs_elasticity", ml)
 
 
+REFERENCE_DIR = os.path.join(HERE, "reference")
+
+
+def adopt_builders():
+    """The reference solvers of test_from_pyamg_adopts_every_solver_family (np.random.seed(1) before each)."""
+    from pyamg.gallery import advection_2d
+    A2, A3 = poisson((24, 24), format="csr"), poisson((9, 9, 9), format="csr")
+    return {
+        "rs_default": lambda: pyamg.ruge_stuben_solver(A2),
+        "rs_cljp_direct_jacobi": lambda: pyamg.ruge_stuben_solver(
+            A2, CF="CLJP", interpolation="direct", presmoother=("jacobi", {"omega": 0.8}), postsmoother=("jacobi", {"omega": 0.8})),
+        "sa_default": lambda: pyamg.smoothed_aggregation_solver(A3),
+        "sa_elasticity_default": lambda: pyamg.smoothed_aggregation_solver(linear_elasticity((10, 10))[0],
+                                                                        B=linear_elasticity((10, 10))[1]),
+        "sa_energy_chebyshev": lambda: pyamg.smoothed_aggregation_solver(
+            stencil_grid(diffusion_stencil_2d(0.01, np.pi / 4, "FD"), (24, 24), format="csr"), smooth="energy",
+            presmoother=("chebyshev", {"degree": 2}), postsmoother=("chebyshev", {"degree": 2})),
+        "rootnode": lambda: pyamg.rootnode_solver(A2),
+        "pairwise": lambda: pyamg.pairwise_solver(A2),
+        "adaptive_sa": lambda: pyamg.aggregation.adaptive_sa_solver(A2, num_candidates=1)[0],
+        "air": lambda: pyamg.air_solver(advection_2d((20, 20))[0].tocsr()),
+        "sa_sor_none_lu": lambda: pyamg.smoothed_aggregation_solver(A2, presmoother=("sor", {"omega": 1.2}),
+                                                                   postsmoother=None, coarse_solver="lu"),
+        "rs_coarse_gauss_seidel": lambda: pyamg.ruge_stuben_solver(A2, max_coarse=50,
+                                                                   coarse_solver=("gauss_seidel", {"iterations": 3})),
+        "sa_richardson_splu": lambda: pyamg.smoothed_aggregation_solver(A2, presmoother="richardson",
+                                                                       postsmoother="richardson", coarse_solver="splu"),
+        "sa_schwarz": lambda: pyamg.smoothed_aggregation_solver(A2.copy(), presmoother="schwarz", postsmoother="schwarz"),
+        "sa_strength_schwarz": lambda: pyamg.smoothed_aggregation_solver(
+            A2.copy(), strength=("symmetric", {"theta": 0.3}), keep=True, presmoother="strength_based_schwarz",
+            postsmoother=("strength_based_schwarz", {"sweep": "forward"})),
+    }
+
+
+def variant_builders():
+    """The reference solvers of test_adopted_hierarchies_all_solve_variants_match_the_reference."""
+    from pyamg.gallery import advection_2d
+    A2 = poisson((20, 20), format="csr")
+    return {"rs": lambda: pyamg.ruge_stuben_solver(A2),
+            "sa_elasticity": lambda: pyamg.smoothed_aggregation_solver(linear_elasticity((8, 8))[0],
+                                                                       B=linear_elasticity((8, 8))[1]),
+            "air": lambda: pyamg.air_solver(advection_2d((16, 16))[0].tocsr()),
+            "rootnode": lambda: pyamg.rootnode_solver(A2)}
+
+
+def main_reference_checks():
+    """Goldens of the tests that compare with the reference directly, under tests/golden/reference/:
+    adopt_<family>.npz / variants_<family>.npz (hierarchies the reference built + its ml.solve results),
+    mis_colouring.npz (its 'MIS' colours) and compiled_kernels.json (digests of its compiled relaxation.h kernels,
+    which needs oracle/_ref/libamg_ref.so)."""
+    import json
+    import warnings
+    import scipy.sparse as sp
+    sys.path.insert(0, os.path.dirname(HERE))
+    import oracle
+    from pyamg_b200.hierarchy_io import load_hierarchy
+    from test_oracle import kernel_digests
+    from test_setup import mis_graphs
+    from test_zz_gpu_widening import ADOPT_FAMILIES, VARIANT_FAMILIES, variant_runs
+    os.makedirs(REFERENCE_DIR, exist_ok=True)
+
+    def load_golden(name):
+        return load_hierarchy(os.path.join(HERE, name + ".npz"))
+
+    builders = adopt_builders()
+    assert sorted(builders) == sorted(ADOPT_FAMILIES)
+    for family in ADOPT_FAMILIES:
+        with warnings.catch_warnings():
+            warnings.simplefilter("ignore")
+            np.random.seed(1)
+            ml = builders[family]()
+            b = np.random.default_rng(2).random(ml.levels[0].A.shape[0])
+            extra = {"b": b, "x_V3": ml.solve(b, tol=0, maxiter=3), "x_W2": ml.solve(b, tol=0, maxiter=2, cycle="W")}
+        save_hierarchy(os.path.join(REFERENCE_DIR, f"adopt_{family}.npz"), ml, extra=extra)
+
+    builders = variant_builders()
+    assert sorted(builders) == sorted(VARIANT_FAMILIES)
+    for family in VARIANT_FAMILIES:
+        with warnings.catch_warnings():
+            warnings.simplefilter("ignore")
+            np.random.seed(1)
+            ml = builders[family]()
+            n = ml.levels[0].A.shape[0]
+            b, x0 = np.random.default_rng(2).random(n), np.random.default_rng(3).random(n)
+            extra = {"b": b, "x0": x0}
+            runs = variant_runs(x0)
+            info, nres = np.full(len(runs), -99), np.zeros(len(runs), dtype=int)
+            for k, kw in enumerate(runs):
+                if family == "air" and kw.get("accel") == "cg":
+                    continue                                  # nonsymmetric operator
+                res = []
+                extra[f"x_{k}"], info[k] = ml.solve(b, residuals=res, return_info=True, **kw)
+                nres[k] = len(res)
+            extra.update(info=info, nres=nres)
+        save_hierarchy(os.path.join(REFERENCE_DIR, f"variants_{family}.npz"), ml, extra=extra)
+
+    # 'MIS' colours of every level of the reference's RS hierarchies on poisson((30, 30)) and poisson((12, 12, 12)),
+    # which are the cfg1 and cfg3 goldens' levels, and of a random symmetric graph
+    R = sp.random(300, 300, 0.03, random_state=1)
+    R = (R + R.T).tocsr()
+    R.sort_indices()
+    z = {"random_indptr": R.indptr.astype(np.int32), "random_indices": R.indices.astype(np.int16)}
+    ref_graphs = []
+    for A in (poisson((30, 30), format="csr"), poisson((12, 12, 12), format="csr")):
+        ref_graphs += [lvl.A for lvl in pyamg.ruge_stuben_solver(A, max_coarse=10).levels]
+    ref_graphs.append(R)
+    graphs = mis_graphs(load_golden, z)
+    assert len(graphs) == len(ref_graphs)
+    for k, (G, Gr) in enumerate(zip(graphs, ref_graphs)):
+        G, Gr = sp.csr_array(G), sp.csr_array(Gr)
+        G.sort_indices()
+        Gr.sort_indices()
+        assert np.array_equal(G.indptr, Gr.indptr) and np.array_equal(G.indices, Gr.indices), k
+        z[f"colours_{k}"] = vertex_coloring(Gr, "MIS").astype(np.uint8)
+    np.savez_compressed(os.path.join(REFERENCE_DIR, "mis_colouring.npz"), **z)
+
+    assert oracle.have_ref(), "oracle/_ref/libamg_ref.so is needed for compiled_kernels.json"
+    from conftest import GOLDEN_ALL
+    digests = {name: kernel_digests(load_golden(name)[0], "ref") for name in GOLDEN_ALL}
+    with open(os.path.join(REFERENCE_DIR, "compiled_kernels.json"), "w") as f:
+        json.dump(digests, f, indent=1)
+        f.write("\n")
+    for fn in sorted(os.listdir(REFERENCE_DIR)):
+        print(f"reference/{fn}: {os.path.getsize(os.path.join(REFERENCE_DIR, fn)) / 1024:.0f} KB")
+
+
 if __name__ == "__main__":
+    if "--reference-checks" in sys.argv:
+        main_reference_checks()
+        sys.exit(0)
     if "--only" in sys.argv:
         ONLY = sys.argv[sys.argv.index("--only") + 1]
     if "--krylov" in sys.argv:

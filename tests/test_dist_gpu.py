@@ -23,7 +23,7 @@ def _ngpus():
 @pytest.mark.parametrize("mode", [("peer",), ("peer", "graph"), ("allgather",)])
 def test_two_gpu_cycle_matches_the_oracle(mode):
     if os.environ.get("AMGB_TEST_EMU") == "1" or _ngpus() < 2:
-        pytest.skip("needs two CUDA devices (gpurun --gpus 2)")
+        pytest.skip("needs two CUDA devices")
     s = socket.socket()
     s.bind(("127.0.0.1", 0))
     port = s.getsockname()[1]

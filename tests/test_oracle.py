@@ -2,16 +2,20 @@
 
 Three anchors (task section 3): the reference's own known-answer vectors restated from
 pyamg/relaxation/tests/test_relaxation.py; golden fixtures produced by running the real reference
-(tests/golden/make_golden.py); and, when oracle/_ref/libamg_ref.so is present, the reference's
-compiled relaxation.h itself.  The oracle restates the reference's arithmetic in the same order,
+(tests/golden/make_golden.py); and digests of what the reference's compiled relaxation.h
+returned on seeded inputs (tests/golden/reference/).  The oracle restates the reference's arithmetic in the same order,
 so agreement is expected to rounding of identical operations (bit-exact in practice).
 """
+import hashlib
+import json
+import os
+
 import numpy as np
 import pytest
 import scipy.sparse as sp
 
 import oracle
-from conftest import GOLDEN_ALL as GOLDEN, relerr
+from conftest import GOLDEN_ALL as GOLDEN, GOLDEN_DIR, relerr
 
 TIGHT = 1e-14   # oracle vs reference: same operations, same order
 
@@ -156,15 +160,42 @@ def test_oracle_kernels_match_reference(name, load_golden):
 
 
 # ---------------------------------------------------------------- compiled reference cross-check
-@pytest.mark.skipif(not oracle.have_ref(), reason="oracle/_ref/libamg_ref.so not built")
+COMPILED_KERNELS = os.path.join(GOLDEN_DIR, "reference", "compiled_kernels.json")
+
+
+def kernel_digests(ml, kernels):
+    """Per level, the SHA-256 of what one application of every kernel a cycle uses there returns on seeded vectors:
+    pre- and post-smoother, A x, R x, P x_c and a coarsest-level relaxation.  Only native kernels and SciPy's sparse
+    matvecs take part (no BLAS), so the digests do not depend on the host CPU."""
+    out = []
+    for k, d in enumerate(oracle.hierarchy_spec(ml)):
+        rng = np.random.default_rng(1000 + k)
+        A = d["A"]
+        x, b = rng.random(A.shape[0]), rng.random(A.shape[0])
+        h = hashlib.sha256()
+        for which in ("pre", "post", "coarse_relax"):
+            if which in d:
+                y = x.copy()
+                oracle._smooth(d[which], A, y, b, kernels)
+                h.update(y.tobytes())
+        h.update(oracle.matvec(A, x, kernels).tobytes())
+        if "P" in d:
+            h.update(oracle.matvec(d["R"], x, kernels).tobytes())
+            h.update(oracle.matvec(d["P"], rng.random(d["P"].shape[1]), kernels).tobytes())
+        out.append(h.hexdigest())
+    return out
+
+
 @pytest.mark.parametrize("name", GOLDEN)
 def test_oracle_equals_compiled_reference(name, load_golden):
-    """The C restatement and the reference's own relaxation.h (+ SciPy matvec) agree bit for bit."""
-    ml, ex = load_golden(name)
-    spec = oracle.hierarchy_spec(ml)
-    a = oracle.Cycle(spec, coarse_pinv=ml.coarse_solver.P, kernels="oracle").solve(ex["b"], tol=0, maxiter=3)
-    r = oracle.Cycle(spec, coarse_pinv=ml.coarse_solver.P, kernels="ref").solve(ex["b"], tol=0, maxiter=3)
-    assert np.array_equal(a, r)
+    """The C restatement and the reference's own relaxation.h (+ SciPy matvec) agree bit for bit: the oracle's
+    kernels against digests of what oracle/_ref/libamg_ref.so returned on the same inputs
+    (tests/golden/reference/, written by make_golden.py --reference-checks)."""
+    ml, _ = load_golden(name)
+    with open(COMPILED_KERNELS) as f:
+        want = json.load(f)[name]
+    got = kernel_digests(ml, "oracle")
+    assert got == want, [k for k, (g, w) in enumerate(zip(got, want)) if g != w]
 
 
 @pytest.mark.parametrize("name", GOLDEN)

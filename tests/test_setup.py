@@ -1,6 +1,8 @@
 """CPU tests of the host-side setup (pyamg_b200.classical / gallery / graph): the hierarchies it
 builds coincide with the ones the REAL reference built (golden fixtures), so bench inputs generated
 on the GPU box are the BASELINE configs' hierarchies."""
+import os
+
 import numpy as np
 import pytest
 
@@ -198,18 +200,27 @@ def test_vector_sa_setup_reproduces_reference_elasticity_hierarchy(load_golden):
     assert ml3.levels[0].B.shape == (392, 2) and ml3.levels[1].A.blocksize == (2, 2)
 
 
-def test_mis_colouring_is_the_references():
-    """pyamg.graph.vertex_coloring(G, 'MIS') (amg_core/graph.h:218-235: repeated lexicographically-first maximal
-    independent sets) equals natural-order first fit vertex by vertex -- checked against the REAL reference (installed
-    by oracle/build.py into baseline/_ref) on every level of two Ruge-Stuben hierarchies and a random graph."""
-    pyamg = pytest.importorskip("pyamg")
+MIS_COLOURS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference", "mis_colouring.npz")
+
+
+def mis_graphs(load_golden, z):
+    """Every level of the Ruge-Stuben hierarchies the REAL reference built for poisson((30, 30)) and
+    poisson((12, 12, 12)) (golden cfg1 and cfg3), then a random symmetric graph stored beside the colours."""
     import scipy.sparse as sp
-    from pyamg.graph import vertex_coloring as reference_coloring
+    graphs = [lvl.A for name in ("cfg1_rs_gs_poisson2d", "cfg3_rs_mcgs_poisson3d") for lvl in load_golden(name)[0].levels]
+    n = len(z["random_indptr"]) - 1
+    graphs.append(sp.csr_array((np.ones(len(z["random_indices"])), z["random_indices"], z["random_indptr"]), shape=(n, n)))
+    return graphs
+
+
+def test_mis_colouring_is_the_references(load_golden):
+    """pyamg.graph.vertex_coloring(G, 'MIS') (amg_core/graph.h:218-235: repeated lexicographically-first maximal
+    independent sets) equals natural-order first fit vertex by vertex -- checked against the colours the REAL
+    reference computed (tests/golden/reference/mis_colouring.npz) on every level of two Ruge-Stuben hierarchies and
+    a random graph."""
     from pyamg_b200.graph import vertex_coloring
-    graphs = []
-    for A in (pyamg.gallery.poisson((30, 30), format="csr"), pyamg.gallery.poisson((12, 12, 12), format="csr")):
-        graphs += [lvl.A for lvl in pyamg.ruge_stuben_solver(A, max_coarse=10).levels]
-    R = sp.random(300, 300, 0.03, random_state=1)
-    graphs.append((R + R.T).tocsr())
-    for G in graphs:
-        assert np.array_equal(reference_coloring(G, "MIS"), vertex_coloring(G, "MIS"))
+    z = np.load(MIS_COLOURS)
+    graphs = mis_graphs(load_golden, z)
+    assert len(graphs) == len([k for k in z.files if k.startswith("colours_")])
+    for k, G in enumerate(graphs):
+        assert np.array_equal(z[f"colours_{k}"], vertex_coloring(G, "MIS")), k

@@ -7,6 +7,8 @@ far only run on tests/emu (the engine's kernel sources on host fibers: `AMGB_TES
 
 Tolerance as everywhere: ||x_gpu - x_ref|| / ||x_ref|| < 1e-12 in fp64 (1e-11 for the Krylov-accelerated runs).
 """
+import os
+
 import numpy as np
 import pytest
 import scipy.sparse as sp
@@ -586,89 +588,54 @@ def random_hierarchy_check(case, monkeypatch, envs):
         assert relerr(ml.solve(b, tol=0, maxiter=2), xo) < 1e-12, env
 
 
-# ------------------------------------------------------------------ adoption of real reference solvers (needs pyamg)
-@pytest.mark.parametrize("family", ["rs_default", "rs_cljp_direct_jacobi", "sa_default", "sa_elasticity_default",
-                                    "sa_energy_chebyshev", "rootnode", "pairwise", "adaptive_sa", "air",
-                                    "sa_sor_none_lu", "rs_coarse_gauss_seidel", "sa_richardson_splu", "sa_schwarz",
-                                    "sa_strength_schwarz"])
+# ------------------------------------------------------------------ adoption of real reference solvers
+# The hierarchies are the ones the REAL reference built (tests/golden/make_golden.py --reference-checks writes each
+# with pyamg_b200.hierarchy_io.save_hierarchy, i.e. through the same reading of its smoothers and coarse solver that
+# from_pyamg does, next to the reference's own ml.solve results on them).
+ADOPT_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference")
+ADOPT_FAMILIES = ["rs_default", "rs_cljp_direct_jacobi", "sa_default", "sa_elasticity_default", "sa_energy_chebyshev",
+                  "rootnode", "pairwise", "adaptive_sa", "air", "sa_sor_none_lu", "rs_coarse_gauss_seidel",
+                  "sa_richardson_splu", "sa_schwarz", "sa_strength_schwarz"]
+VARIANT_FAMILIES = ["rs", "sa_elasticity", "air", "rootnode"]
+
+
+def variant_runs(x0):
+    """The ml.solve arguments of test_adopted_hierarchies_all_solve_variants_match_the_reference, in order."""
+    return (dict(accel="cg", tol=1e-8, maxiter=8), dict(accel="gmres", tol=1e-8, maxiter=8),
+            dict(accel="fgmres", tol=1e-8, maxiter=8, cycle="W"), dict(accel="bicgstab", tol=1e-8, maxiter=8),
+            dict(accel="fgmres", cycle="AMLI", tol=1e-6, maxiter=4), dict(tol=1e-6, maxiter=30, x0=x0),
+            dict(cycle="AMLI", tol=0, maxiter=2), dict(cycle="F", tol=0, maxiter=2, cycles_per_level=2))
+
+
+@pytest.mark.parametrize("family", ADOPT_FAMILIES)
 def test_from_pyamg_adopts_every_solver_family(family):
-    """MultilevelSolver.from_pyamg on hierarchies the REAL reference builds (skipped where pyamg is not importable,
-    i.e. on the GPU box; in the build container: PYTHONPATH=<reference build> AMGB_TEST_EMU=1 pytest -m gpu -k adopts):
-    three V-cycles and two W-cycles equal the reference's own ml.solve to 1e-12 -- classical RS (RS / CLJP
-    splittings, direct interpolation), SA with default block Gauss-Seidel (scalar and elasticity), energy-minimising
-    SA + Chebyshev, root-node, pairwise, adaptive SA, AIR, SOR on BSR coarse levels (omega ignored there, as in the
-    reference), None smoothers, lu / splu / relaxation coarse solvers."""
-    pyamg = pytest.importorskip("pyamg")
-    import warnings
-    from pyamg.gallery import poisson, linear_elasticity, advection_2d, stencil_grid
-    from pyamg.gallery.diffusion import diffusion_stencil_2d
-    A2, A3 = poisson((24, 24), format="csr"), poisson((9, 9, 9), format="csr")
-    build = {
-        "rs_default": lambda: pyamg.ruge_stuben_solver(A2),
-        "rs_cljp_direct_jacobi": lambda: pyamg.ruge_stuben_solver(
-            A2, CF="CLJP", interpolation="direct", presmoother=("jacobi", {"omega": 0.8}), postsmoother=("jacobi", {"omega": 0.8})),
-        "sa_default": lambda: pyamg.smoothed_aggregation_solver(A3),
-        "sa_elasticity_default": lambda: pyamg.smoothed_aggregation_solver(*[linear_elasticity((10, 10))[k] for k in (0,)],
-                                                                        B=linear_elasticity((10, 10))[1]),
-        "sa_energy_chebyshev": lambda: pyamg.smoothed_aggregation_solver(
-            stencil_grid(diffusion_stencil_2d(0.01, np.pi / 4, "FD"), (24, 24), format="csr"), smooth="energy",
-            presmoother=("chebyshev", {"degree": 2}), postsmoother=("chebyshev", {"degree": 2})),
-        "rootnode": lambda: pyamg.rootnode_solver(A2),
-        "pairwise": lambda: pyamg.pairwise_solver(A2),
-        "adaptive_sa": lambda: pyamg.aggregation.adaptive_sa_solver(A2, num_candidates=1)[0],
-        "air": lambda: pyamg.air_solver(advection_2d((20, 20))[0].tocsr()),
-        "sa_sor_none_lu": lambda: pyamg.smoothed_aggregation_solver(A2, presmoother=("sor", {"omega": 1.2}),
-                                                                   postsmoother=None, coarse_solver="lu"),
-        "rs_coarse_gauss_seidel": lambda: pyamg.ruge_stuben_solver(A2, max_coarse=50,
-                                                                   coarse_solver=("gauss_seidel", {"iterations": 3})),
-        "sa_richardson_splu": lambda: pyamg.smoothed_aggregation_solver(A2, presmoother="richardson",
-                                                                       postsmoother="richardson", coarse_solver="splu"),
-        "sa_schwarz": lambda: pyamg.smoothed_aggregation_solver(A2.copy(), presmoother="schwarz", postsmoother="schwarz"),
-        "sa_strength_schwarz": lambda: pyamg.smoothed_aggregation_solver(
-            A2.copy(), strength=("symmetric", {"theta": 0.3}), keep=True, presmoother="strength_based_schwarz",
-            postsmoother=("strength_based_schwarz", {"sweep": "forward"})),
-    }
-    with warnings.catch_warnings():
-        warnings.simplefilter("ignore")
-        np.random.seed(1)
-        ref = build[family]()
-        b = np.random.default_rng(2).random(ref.levels[0].A.shape[0])
-        gpu = pyamg_b200.MultilevelSolver.from_pyamg(ref)
-        assert relerr(gpu.solve(b, tol=0, maxiter=3), ref.solve(b, tol=0, maxiter=3)) < TOL
-        assert relerr(gpu.solve(b, tol=0, maxiter=2, cycle="W"), ref.solve(b, tol=0, maxiter=2, cycle="W")) < TOL
+    """MultilevelSolver.from_pyamg on hierarchies the REAL reference built: three V-cycles and two W-cycles equal the
+    reference's own ml.solve to 1e-12 -- classical RS (RS / CLJP splittings, direct interpolation), SA with default
+    block Gauss-Seidel (scalar and elasticity), energy-minimising SA + Chebyshev, root-node, pairwise, adaptive SA,
+    AIR, SOR on BSR coarse levels (omega ignored there, as in the reference), None smoothers, lu / splu / relaxation
+    coarse solvers."""
+    from pyamg_b200.hierarchy_io import load_hierarchy
+    ref, ex = load_hierarchy(os.path.join(ADOPT_DIR, f"adopt_{family}.npz"))
+    gpu = pyamg_b200.MultilevelSolver.from_pyamg(ref)
+    assert relerr(gpu.solve(ex["b"], tol=0, maxiter=3), ex["x_V3"]) < TOL
+    assert relerr(gpu.solve(ex["b"], tol=0, maxiter=2, cycle="W"), ex["x_W2"]) < TOL
 
 
-@pytest.mark.parametrize("family", ["rs", "sa_elasticity", "air", "rootnode"])
+@pytest.mark.parametrize("family", VARIANT_FAMILIES)
 def test_adopted_hierarchies_all_solve_variants_match_the_reference(family):
-    """On hierarchies adopted from the real reference (needs pyamg: build container only): CG / GMRES / FGMRES /
-    BiCGStab acceleration, FGMRES + AMLI, tolerance stop from x0, AMLI and F(cycles_per_level=2) cycles -- same
-    iterates, iteration counts and info flags as the reference's own ml.solve."""
-    pyamg = pytest.importorskip("pyamg")
-    import warnings
-    from pyamg.gallery import poisson, linear_elasticity, advection_2d
-    A2 = poisson((20, 20), format="csr")
-    build = {"rs": lambda: pyamg.ruge_stuben_solver(A2),
-             "sa_elasticity": lambda: pyamg.smoothed_aggregation_solver(linear_elasticity((8, 8))[0], B=linear_elasticity((8, 8))[1]),
-             "air": lambda: pyamg.air_solver(advection_2d((16, 16))[0].tocsr()),
-             "rootnode": lambda: pyamg.rootnode_solver(A2)}
-    with warnings.catch_warnings():
-        warnings.simplefilter("ignore")
-        np.random.seed(1)
-        ref = build[family]()
-        gpu = pyamg_b200.MultilevelSolver.from_pyamg(ref)
-        n = ref.levels[0].A.shape[0]
-        b, x0 = np.random.default_rng(2).random(n), np.random.default_rng(3).random(n)
-        for kw in (dict(accel="cg", tol=1e-8, maxiter=8), dict(accel="gmres", tol=1e-8, maxiter=8),
-                   dict(accel="fgmres", tol=1e-8, maxiter=8, cycle="W"), dict(accel="bicgstab", tol=1e-8, maxiter=8),
-                   dict(accel="fgmres", cycle="AMLI", tol=1e-6, maxiter=4), dict(tol=1e-6, maxiter=30, x0=x0),
-                   dict(cycle="AMLI", tol=0, maxiter=2), dict(cycle="F", tol=0, maxiter=2, cycles_per_level=2)):
-            if family == "air" and kw.get("accel") == "cg":
-                continue                                  # nonsymmetric operator
-            rr, rg = [], []
-            xr, ir = ref.solve(b, residuals=rr, return_info=True, **kw)
-            xg, ig = gpu.solve(b, residuals=rg, return_info=True, **kw)
-            assert (ir, len(rr)) == (ig, len(rg)), kw
-            assert relerr(xg, xr) < 1e-9, kw
+    """On hierarchies adopted from the real reference: CG / GMRES / FGMRES / BiCGStab acceleration, FGMRES + AMLI,
+    tolerance stop from x0, AMLI and F(cycles_per_level=2) cycles -- same iterates, iteration counts and info flags
+    as the reference's own ml.solve."""
+    from pyamg_b200.hierarchy_io import load_hierarchy
+    ref, ex = load_hierarchy(os.path.join(ADOPT_DIR, f"variants_{family}.npz"))
+    gpu = pyamg_b200.MultilevelSolver.from_pyamg(ref)
+    for k, kw in enumerate(variant_runs(ex["x0"])):
+        if family == "air" and kw.get("accel") == "cg":
+            continue                                  # nonsymmetric operator
+        rg = []
+        xg, ig = gpu.solve(ex["b"], residuals=rg, return_info=True, **kw)
+        assert (int(ex["info"][k]), int(ex["nres"][k])) == (ig, len(rg)), kw
+        assert relerr(xg, ex[f"x_{k}"]) < 1e-9, kw
 
 
 # ------------------------------------------------------------------ CF / FC block Jacobi (AIR on block systems)
